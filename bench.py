@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- projections/sec on the headline scene (100k Gaussians, 512x512 cone-beam, 50 views).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one forward X-ray projection of the synthetic scene (views cycle through the 50 angles).
@@ -33,6 +33,13 @@ reference arm (--impl reference)
   arm therefore times the UNMODIFIED reference CUDA sources compiled for sm_100a into oracle/_ref/libr2ref.so
   (oracle/build_ref.sh) on the GPU with the identical per-step event / L2-flush protocol; if that library is
   absent it falls back to the CPU oracle port.  Rank 0 only.
+
+--dump-outputs DIR
+  After the timed steps, writes what the last timed step returned to its caller as DIR/image.npy (the [1,H,W]
+  detector image) and, on one GPU, DIR/radii.npy (per-Gaussian screen radii), both float32.  Both GPU arms write the
+  same names.  The scene and the views are seeded, so the same arguments give the same inputs in every run and two
+  builds can be compared output for output.  An array over its share of 64 MiB is replaced by a fixed, seeded
+  sample of its elements (the same positions in every run).
 """
 from __future__ import annotations
 
@@ -80,6 +87,8 @@ def parse_args():
     ap.add_argument("--cpu-baseline-child", default=None, choices=["port", "torch"], help=argparse.SUPPRESS)
     ap.add_argument("--reduce", default="p2p", choices=["p2p", "nccl"],
                     help="N > 1: how the per-rank partial images are summed (NVLink peer-memory kernel | NCCL)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32)")
     return ap.parse_args()
 
 
@@ -194,6 +203,22 @@ def timed_steps(step_fn, steps, warmup, flush_buf, stream_sync):
         stops[i].record()
     stream_sync()
     return [s.elapsed_time(e) for s, e in zip(starts, stops)]
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """arrays: name -> numpy array, written as float32 DIR/<name>.npy; an array over its share of DUMP_LIMIT_BYTES
+    is replaced by a sample of its flattened elements at positions drawn from a fixed seed."""
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // len(arrays) - 4096           # room for the .npy header
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.nbytes > share:
+            idx = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def usable_cores() -> int:
@@ -375,21 +400,28 @@ def run_ours(args, rank, world, local_rank):
         if int(flag.item()) == 0:
             reducer, args.reduce = None, "nccl"
     final = torch.empty((1, H, W), dtype=torch.float32, device=dev)
+    last = {}
 
     def step(i):
         if reducer is not None:
             fwd(i, out=reducer.partial().view(1, H, W))
-            reducer.reduce(final)
+            last["image"] = reducer.reduce(final)
             return
         out = fwd(i)
         if world > 1:
             dist.all_reduce(out, op=dist.ReduceOp.SUM)
+        last["image"] = out
 
     sampler = ClockSampler(local_rank)
     sync()
     with sampler:
         ms = timed_steps(step, args.steps, args.warmup, flush, sync)
     total_ms = float(sum(ms))
+    if args.dump_outputs and rank == 0:     # before the buffers are reused below
+        outputs = {"image": last["image"].cpu().numpy()}
+        if world == 1:
+            outputs["radii"] = eng.radii.cpu().numpy()
+        dump_outputs(args.dump_outputs, outputs)
     # back-to-back (warm L2, launches pipelined) for information; with N > 1 the all-reduce of step i runs on a
     # side stream and overlaps the render of step i+1 (ring of output buffers)
     sync()
@@ -652,6 +684,8 @@ def run_reference(args):
     with sampler:
         ms = timed_steps(step, args.steps, args.warmup, flush, sync)
     total_ms = float(sum(ms))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"image": out.cpu().numpy(), "radii": radii.cpu().numpy()})
     value = args.steps / (total_ms * 1e-3)
     # back-to-back, warm L2
     sync()

